@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- short-term feature_extraction throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] -- 1000 synthetic 16 kHz mono int16 10 s clips per
 GPU, window/step 50/25 ms, full 68-row short-term feature matrix.  One "step" = the whole hot path
@@ -16,6 +16,9 @@ out, copies inside the timed region); `roofline` = algorithmic bytes / kernel ti
 against the measured HBM peak (plus the FP32-issue fraction of the committed ncu capture);
 `cpu_baseline` = the unmodified reference (staged under oracle/_ref by oracle/make_ref.py) on the host
 cores, one single-threaded process per physical core, bounded sample.
+`--dump-outputs DIR` writes the feature matrices of the last timed step (rank 0: the gathered ones) for a fixed, seeded
+sample of DUMP_CLIPS clips as DIR/features.npy (float32 [DUMP_CLIPS, 68, T], 55.6 MB); the clips are generated from fixed
+seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -30,6 +33,7 @@ sys.path.insert(0, ROOT)
 
 FS, WINDOW, STEP, CLIP_SAMPLES, CLIPS_PER_GPU = 16000, 800, 400, 160000, 1000
 FRAMES_PER_CLIP = (CLIP_SAMPLES - WINDOW) // STEP + 1            # 399
+DUMP_CLIPS = 512                                                  # --dump-outputs: 512 x 68 x 399 float32 = 55.6 MB
 ALG_BYTES_PER_CLIP = 2 * CLIP_SAMPLES + 4 * 68 * FRAMES_PER_CLIP   # 428 528 (SURVEY.md 8d)
 METRIC = "audio frames/sec short-term feature_extraction @16kHz 50/25ms"
 WORKLOAD = "1000 synthetic 16 kHz mono int16 10 s clips per GPU, win/step 50/25 ms, 68 short-term features (BASELINE configs[1])"
@@ -243,7 +247,7 @@ def ncu_facts():
 def run_reference(args, rank, world):
     if rank != 0:
         return
-    steps = max(1, args.steps)
+    steps = args.steps
     cb, frames, dt = cpu_baseline(target_seconds=30.0, steps=steps, warmup=min(args.warmup, 3))
     line = {"impl": "reference", "metric": METRIC, "value": cb["value"], "unit": "frames/s", "n_gpus": args.gpus,
             "steps": steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / steps, "higher_is_better": True, "scaling": "weak",
@@ -256,6 +260,12 @@ def run_reference(args, rank, world):
 
 
 # ----------------------------------------------------------------------------- our arm
+def dump_clips(n_clips):
+    """Indices of the clips --dump-outputs writes: a fixed, seeded sample (the same for every build)."""
+    import numpy as np
+    return np.sort(np.random.default_rng(0).choice(n_clips, DUMP_CLIPS, replace=False))
+
+
 def synth_device_batch(torch, n_clips, seed, device):
     """Noise + three harmonics per clip, generated on the device (SURVEY.md 8d recipe, bulk variant)."""
     g = torch.Generator(device=device)
@@ -362,11 +372,18 @@ def run_ours(args, rank, world, local_rank):
     with ClockSampler(local_rank) as clk:
         ms_total, kernel_ms = timed(main_mode, args.steps)
         launches = L.b200aa_launch_count() - launches0          # our kernels launched inside the timed region
+        if args.dump_outputs and rank == 0:                     # taken before any later call writes the buffer again
+            last = gathers[(args.steps - 1) % 2].view(0, world * B) if world > 1 else local_out
+            dump = last.index_select(0, torch.from_numpy(dump_clips(world * B)).to(dev))
         # keep the sampler alive for a few more identical steps if the timed region was very short
         t_end = time.time() + 0.25
         while time.time() < t_end and len(clk.samples) < 8:
             pkg.feature_extraction_batch(clips, FS, WINDOW, STEP, deltas=True, out=local_out, plan=plan)
             torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "features.npy"), dump.cpu().numpy())
     ms_per_step = ms_total / args.steps
     frames_per_step = world * B * T
     value = frames_per_step / (ms_per_step * 1e-3)
@@ -460,6 +477,10 @@ def run_ours(args, rank, world, local_rank):
             "clocks": clk.summary(), "e2e": e2e, "gpu_launches": int(launches)}
     if scaling_detail:
         line["scaling_detail"] = scaling_detail
+    if args.dump_outputs:
+        line["dump_outputs"] = {"features.npy": {"shape": [DUMP_CLIPS, 68, T], "dtype": "float32",
+                                                 "clips": "numpy.random.default_rng(0).choice(%d, %d, replace=False), sorted"
+                                                          % (world * B, DUMP_CLIPS)}}
     if world == 1 and not args.no_cpu:
         if full_affinity is not None:
             os.sched_setaffinity(0, full_affinity)       # the CPU baseline uses every core of the box, not only the GPU's node
@@ -477,7 +498,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg (profiling runs)")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-pipeline leg (profiling runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's features (seeded sample of clips) to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's outputs (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

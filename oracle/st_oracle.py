@@ -10,9 +10,9 @@ here against golden vectors produced by the unmodified reference
 ``oracle/make_golden.py``; fixtures: ``tests/golden/*.npz``).  The reference's
 own tests pin shapes only (pytests/test_feature_extraction.py:14-15,27-28;
 those shape pins are reproduced in ``tests/test_oracle_golden.py::
-test_reference_pytest_inputs``).  ``tests/test_oracle_vs_reference.py`` additionally runs the oracle against the
-imported reference on randomised configurations and error cases wherever the
-reference tree is present.
+test_reference_pytest_inputs``).  ``tests/test_oracle_vs_reference.py`` additionally holds the oracle to
+the reference's values on randomised configurations and error cases
+(``tests/golden/vs_reference.npz``, generator ``oracle/make_golden_vs_reference.py``).
 
 Third-party arithmetic: the reference takes its DFT and DCT from SciPy
 (``scipy.fftpack.fft`` ShortTermFeatures.py:5,617 and

@@ -134,7 +134,7 @@ def test_mid_awkward_ratio(P, golden_synth):
 ])
 def test_error_precedence(P, fs, w, s, n, exc, text):
     """Exception types of the unmodified reference on these inputs (tests/test_oracle_vs_reference.py checks
-    the oracle against it where the reference tree exists)."""
+    the oracle against the reference's stored values)."""
     x = O.synth_clip(1, n, fs)
     for fn in (lambda: P.ShortTermFeatures.feature_extraction(x, fs, w, s),
                lambda: P.MidTermFeatures.mid_feature_extraction(x, fs, 4 * w, 4 * w, w, s)):

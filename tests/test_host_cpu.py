@@ -2,7 +2,6 @@
 values of the unmodified reference, and the file decoders (WAV layout walk, direct-into-buffer decode, AIFF, stereo)."""
 import os
 import struct
-import sys
 import wave
 
 import numpy as np
@@ -13,36 +12,56 @@ from tests.conftest import load_golden
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+BEAT_ROWS = 19          # beat_extraction reads short-term rows 0-18 only (reference MidTermFeatures.py:31-32)
+
+
+def beat_walks():
+    """Random-walk feature matrices 4-7 of tests/golden/beat.npz, regenerated from their seed."""
+    rng = np.random.default_rng(9)
+    return [np.cumsum(rng.standard_normal((68, 300 + 40 * i)), axis=1) * 0.05 + rng.standard_normal((68, 1)) for i in range(4, 8)]
+
+
+def peak_inputs():
+    """Seeded (signal, peakdet threshold, feature matrix) triples of test_beat_extraction_against_imported_reference."""
+    rng = np.random.default_rng(3)
+    out = []
+    for k in range(6):
+        v = np.cumsum(rng.standard_normal(400)) * (0.1 + k)
+        delta = 2.0 * np.abs(np.diff(v)).mean()
+        out.append((v, delta, np.cumsum(rng.standard_normal((34, 200 + 30 * k)), axis=1)))
+    return out
+
+
 def test_beat_extraction_matches_reference_golden():
     """tests/golden/beat.npz: MidTermFeatures.beat_extraction of the unmodified reference (oracle/make_golden_r2.py;
-    numpy.Inf / numpy.NaN aliased for NumPy 2) on 8 feature matrices."""
+    numpy.Inf / numpy.NaN aliased for NumPy 2) on 8 feature matrices: the short-term features of four pulse clips (rows
+    0-18 stored, the others zero) and four seeded random walks."""
     from pyaudioanalysis_b200.MidTermFeatures import beat_extraction
     g = load_golden("beat.npz")
+    walks = beat_walks()
     for i in range(int(g["n"])):
-        bpm, ratio = beat_extraction(g["st_%d" % i], float(g["win_%d" % i]))
+        if i < 4:
+            st = np.zeros((68, g["st_%d" % i].shape[1]))
+            st[:BEAT_ROWS] = g["st_%d" % i]
+        else:
+            st = walks[i - 4]
+            assert st.sum() == pytest.approx(float(g["sum_%d" % i]), rel=1e-12), "random walk %d is not the golden input" % i
+        bpm, ratio = beat_extraction(st, float(g["win_%d" % i]))
         assert bpm == pytest.approx(float(g["bpm_%d" % i]), rel=1e-12), i
         assert ratio == pytest.approx(float(g["ratio_%d" % i]), rel=1e-12, abs=1e-15), i
 
 
 def test_beat_extraction_against_imported_reference():
-    from oracle.ref_import import reference_available, load_reference
-    if not reference_available():
-        pytest.skip("reference tree not present")
-    S, M, A = load_reference()
-    if not hasattr(np, "Inf"):
-        np.Inf, np.NaN = np.inf, np.nan
+    """Peak picking and beat_extraction against the reference's utilities.peakdet / MidTermFeatures.beat_extraction on
+    seeded inputs (values in tests/golden/beat.npz, oracle/make_golden_r2.py)."""
     from pyaudioanalysis_b200.MidTermFeatures import beat_extraction, _peak_positions
-    U = sys.modules["pyAudioAnalysis.utilities"]
-    rng = np.random.default_rng(3)
-    for k in range(6):
-        v = np.cumsum(rng.standard_normal(400)) * (0.1 + k)
-        delta = 2.0 * np.abs(np.diff(v)).mean()
-        assert _peak_positions(v, delta) == [int(p) for p in U.peakdet(v, delta)[0]]
-        st = np.cumsum(rng.standard_normal((34, 200 + 30 * k)), axis=1)
-        for win in (0.05, 0.025, 0.1):
-            assert beat_extraction(st, win) == pytest.approx(M.beat_extraction(st, win), rel=1e-12)
+    g = load_golden("beat.npz")
+    for k, (v, delta, st) in enumerate(peak_inputs()):
+        assert _peak_positions(v, delta) == g["peaks_%d" % k].tolist()
+        for win, ref in zip((0.05, 0.025, 0.1), g["beats_%d" % k]):
+            assert beat_extraction(st, win) == pytest.approx(tuple(ref), rel=1e-12)
     flat = np.ones((34, 100))
-    assert beat_extraction(flat, 0.05) == pytest.approx(M.beat_extraction(flat, 0.05))
+    assert beat_extraction(flat, 0.05) == pytest.approx(tuple(g["beats_flat"]))
 
 
 def _write_wav(path, data, fs, extra_chunk=False):
