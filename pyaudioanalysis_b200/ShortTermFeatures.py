@@ -34,8 +34,11 @@ def feature_names(deltas=True):
 def _as_clip(signal):
     """1-D host array in one of the two device sample formats.
 
-    int16 stays int16 (exact).  Everything else becomes float32: the path is invariant to the
-    input scale (the reference divides by 2**15 and then by the clip's max |x - mean|).
+    int16 stays int16 (exact).  Everything else becomes float32.  The reference divides by 2**15
+    and then by max |x/2**15 - mean| + 1e-10, so the features do not depend on the input scale
+    as long as the clip's largest excursion from its mean is far above 2**15 * 1e-10 (about
+    3.3e-6; at 1e-6 the energy row drops by an order of magnitude).  Quieter float clips keep
+    the reference's scale dependence, and the GPU path reproduces it.
     """
     x = np.asarray(signal)
     if x.ndim != 1:

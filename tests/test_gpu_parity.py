@@ -384,12 +384,15 @@ def test_kernel_kinds_agree(P):
 
 
 def test_row_kernels_agree(P):
-    """spectrogram / chromagram through the default kernel (solo for 882 / 400 / 600, CTA for 800), the CTA kernel, the
-    generic kernel, and the oracle."""
+    """spectrogram / chromagram through the default kernel (solo for 882 / 400 / 600, CTA for 800 / 320 / 480 / 640,
+    generic for the pair-only windows 512 / 960 / 1024), the CTA kernel where the window has one, the generic kernel,
+    and the oracle."""
     import torch
     from pyaudioanalysis_b200._lib import Plan
     for fs, w, s, n in [(16000, 800, 400, 40000), (44100, 882, 441, 50000), (16000, 800, 800, 24000), (16000, 800, 200, 16400),
-                        (16000, 400, 160, 16000), (8000, 600, 300, 12000), (44100, 882, 882, 30000), (44100, 882, 300, 20001)]:
+                        (16000, 400, 160, 16000), (8000, 600, 300, 12000), (44100, 882, 882, 30000), (44100, 882, 300, 20001),
+                        (16000, 320, 160, 12000), (16000, 480, 240, 12000), (16000, 640, 320, 16000),
+                        (16000, 512, 256, 16000), (48000, 960, 480, 48000), (16000, 1024, 512, 16000)]:
         clips = np.stack([O.synth_clip(60 + i, n, fs) for i in range(3)])
         d = torch.from_numpy(clips).cuda()
         plans = [Plan(fs, w, s), Plan(fs, w, s).prefer_kernel(1), Plan(fs, w, s)]
@@ -399,7 +402,7 @@ def test_row_kernels_agree(P):
             for pl, what in zip(plans, ("default", "CTA", "generic")):
                 a = fn(d, fs, w, s, plan=pl).cpu().numpy()
                 for i in range(3):
-                    check_close(a[i], refs[i], f"{fn.__name__} {what} kernel fs={fs} w={w} s={s}", atol=atol)
+                    check_close(a[i], refs[i], f"{fn.__name__} {what} plan (kind {pl.kernel_kind()}) fs={fs} w={w} s={s}", atol=atol)
     # a clipped last frame shorter than num_fft makes the reference's scatter raise ValueError (:288)
     bad = O.synth_clip(60, 16300, 16000)
     with pytest.raises(ValueError):
