@@ -58,9 +58,12 @@ template <int R>
 struct PairShape {
     static constexpr int N = 32 * R, K = N / 2, Kp = DenseShape<K>::Kp, C = Kp / 32;
     static constexpr int JK = (K + 31) / 32;         // strided rows that hold real bins (k = lane + 32 j)
-    static constexpr int LS = 34;                    // row stride (floats) of the two transposed pass-1 planes (re, im): even, so the
-                                                     // second pass reads (n2, n2 + 1) pairs as aligned 8-byte words, conflict-free per half-warp
-    static constexpr int TZ = (R * LS > N + 2) ? R * LS : N + 2;   // float2 elements of the transform buffer
+    // pass-1 outputs, row k1: quad m = n2 / 2 holds (re n2, re n2 + 1, im n2, im n2 + 1) -- re and im swap places in quads
+    // 8..15 -- so that the second pass reads the (even, odd) FP32x2 operands of fft32_soa as one 16-byte word per quad.
+    // Row stride LS = 68 floats (4 mod 32 words): the eight rows of a quarter-warp's 16-byte reads hit eight distinct bank
+    // quads; the swap puts lanes n2 and n2 + 16 of pass 1's 4-byte stores on different banks.
+    static constexpr int LS = 68;
+    static constexpr int TZ = (R * LS / 2 > N + 2) ? R * LS / 2 : N + 2;   // float2 elements of the transform buffer
     static constexpr int Lt = N / 10;                // energy-entropy block length (ShortTermFeatures.py:41)
     static constexpr bool kShareable = (N % 160) == 0;    // half a frame = 5 whole blocks, rows split at lane 0 / 16 only
     // after the separation the transform buffer holds the |X| row of frame a (Kp floats) and, behind it, the mel scratch:
@@ -73,14 +76,14 @@ struct PairShape {
     static constexpr int PT0 = RB0 + Kp;                     // spectral-entropy parts of the dense pass (2 x 32)
     static constexpr int CH0 = PT0 + 64;                     // raw chroma sums (2 x 12)
     static_assert(2 * TZ >= CH0 + 24, "|X| rows of both frames + mel scratch + parts + chroma fit the transform buffer");
-    static_assert((RB0 % 4) == 0, "aligned |X| row");
+    static_assert((RB0 % 4) == 0 && (LS % 4) == 0, "aligned |X| row, aligned pass-1 quads");
     static_assert(Lt >= 32, "a 32-sample row touches two blocks at most");
 };
 
 template <int R>
 struct alignas(16) PairWarpMem {
     using S = PairShape<R>;
-    float2 tz[S::TZ];                       // pass-1 outputs, planes re[k1][LS] | im[k1][LS]  ->  Z[k] (natural order, Z[N] = Z[0])  ->
+    float2 tz[S::TZ];                       // pass-1 outputs [k1][LS] (PairShape::LS)  ->  Z[k] (natural order, Z[N] = Z[0])  ->
                                             // |X| row of a | mel scratch | |X| row of b | entropy parts | chroma sums (PairShape::MS0 ...)
     alignas(16) float rowp[S::Kp];          // |X| row of the previous pair's frame b (the flux of frame a needs it)
     float fv[9 * kFvStride];                // feature rows: row 0 = the frame before the tile, rows 1..8 = the tile
@@ -365,6 +368,24 @@ struct TdShape {
     static_assert(FULL || S::kShareable, "half-frame sharing needs whole blocks per half");
 };
 
+// Sign flips of the rows [ZROW0, R) from their ballot masks, one row per lane: lane r holds row r's mask m (0 in a lane
+// that owns no row), takes row r - 1's by one shuffle and counts the pairs (n - 1, n), n >= max(1, NFIRST), of its row.
+// Returns the lane's count plus, in bits 12.., the flip at sample NFIRST (the link between the halves; !FULL only).
+// Whatever lane ZROW0 receives as its predecessor is masked out: its bit 0 is sample 0 (FULL) or precedes NFIRST.
+template <int R, bool FULL>
+__device__ __forceinline__ unsigned td_row_flips(unsigned m, int lane)
+{
+    using Td = TdShape<R, FULL>;
+    const unsigned prev = __shfl_up_sync(0xffffffffu, m, 1);
+    const int nstart = FULL ? 1 : Td::NFIRST, n0 = 32 * lane;
+    const unsigned valid = lane < Td::ROW0 || lane >= R ? 0u
+                         : (n0 >= nstart ? 0xffffffffu : (0xffffffffu << (nstart - n0)));
+    const unsigned c = (m ^ __funnelshift_l(prev, m, 1)) & valid;
+    unsigned v = __popc(c);
+    if (!FULL && lane == Td::ROW0) v += ((c >> Td::LANE0) & 1u) << 12;
+    return v;
+}
+
 template <int R, bool FULL, bool TWO>
 __device__ __forceinline__ void td_frame(const float (&u)[R], float cm, const b200aa_clip_norm &nm, int lane,
                                          float *e /* [NE] */, int &flips, int &link)
@@ -372,29 +393,16 @@ __device__ __forceinline__ void td_frame(const float (&u)[R], float cm, const b2
     using S = PairShape<R>;
     using Td = TdShape<R, FULL>;
     constexpr int N = S::N, Lt = S::Lt;
-    unsigned prevP = 0u, prevQ = 0u;
-    int fl = 0, lk = 0;
+    unsigned mP = 0u, mQ = 0u;          // row `lane`'s sign masks
 #pragma unroll
     for (int r = Td::ZROW0; r < R; ++r) {
         const float d = u[r] - cm;
         // ---- sign masks: P = samples above the clip mean, Q = below (complementary unless a sample can equal the mean)
         const unsigned P = __ballot_sync(0xffffffffu, d > nm.lo);
-        unsigned Q = 0u;
-        if (TWO) Q = __ballot_sync(0xffffffffu, d < nm.hi);
-        if (FULL && r == 0) { prevP = (P & 1u) << 31; prevQ = (Q & 1u) << 31; }      // sample 0 has no predecessor
+        if (lane == r) mP = P;
+        if (TWO) { const unsigned Q = __ballot_sync(0xffffffffu, d < nm.hi); if (lane == r) mQ = Q; }
         if (r >= Td::ROW0) {
             const int n0 = 32 * r;
-            // pairs (n - 1, n) counted for n >= max(1, NFIRST)
-            const int nstart = FULL ? 1 : Td::NFIRST;
-            const unsigned valid = n0 >= nstart ? 0xffffffffu : (n0 + 32 <= nstart ? 0u : (0xffffffffu << (nstart - n0)));
-            const unsigned cP = (P ^ __funnelshift_l(prevP, P, 1)) & valid;
-            fl += __popc(cP);
-            if (!FULL && r == Td::ROW0) lk += int((cP >> Td::LANE0) & 1u);
-            if (TWO) {
-                const unsigned cQ = (Q ^ __funnelshift_l(prevQ, Q, 1)) & valid;
-                fl += __popc(cQ);
-                if (!FULL && r == Td::ROW0) lk += int((cQ >> Td::LANE0) & 1u);
-            }
             // ---- energy of the normalised samples into the row's block(s)
             // (fused multiply-adds, predicated: bit-identical to td_pair below, whichever of the two handles a frame)
             const float y = fmaf(nm.a, d, nm.bp);
@@ -411,8 +419,11 @@ __device__ __forceinline__ void td_frame(const float (&u)[R], float cm, const b2
                 if (i1 >= 0 && i1 < Td::NE) { if (live && !first) e[i1] = fmaf(y, y, e[i1]); }
             }
         }
-        prevP = P; prevQ = Q;
     }
+    unsigned v = td_row_flips<R, FULL>(mP, lane);
+    if (TWO) v += td_row_flips<R, FULL>(mQ, lane);
+    v = __reduce_add_sync(0xffffffffu, v);
+    const int fl = int(v & 0xfffu), lk = int(v >> 12);
     // one-sided counting saw every change once; |s_n - s_(n-1)| is 2 for a sign change without a zero in between
     flips = TWO ? fl : 2 * fl;
     link = TWO ? lk : 2 * lk;
@@ -427,28 +438,19 @@ __device__ __forceinline__ void td_pair(const float2 (&u)[R], float cm, const b2
     using S = PairShape<R>;
     using Td = TdShape<R, FULL>;
     constexpr int N = S::N, Lt = S::Lt;
-    unsigned pPa = 0u, pQa = 0u, pPb = 0u, pQb = 0u;
-    int fa = 0, la = 0, fb = 0, lb = 0;
+    unsigned mPa = 0u, mQa = 0u, mPb = 0u, mQb = 0u;       // row `lane`'s sign masks
     const float2 ncm = make_float2(-cm, -cm), a2 = make_float2(nm.a, nm.a), bp2 = make_float2(nm.bp, nm.bp);
 #pragma unroll
     for (int r = Td::ZROW0; r < R; ++r) {
         const float2 d = __fadd2_rn(u[r], ncm);
         const unsigned Pa = __ballot_sync(0xffffffffu, d.x > nm.lo), Pb = __ballot_sync(0xffffffffu, d.y > nm.lo);
-        unsigned Qa = 0u, Qb = 0u;
-        if (TWO) { Qa = __ballot_sync(0xffffffffu, d.x < nm.hi); Qb = __ballot_sync(0xffffffffu, d.y < nm.hi); }
-        if (FULL && r == 0) { pPa = (Pa & 1u) << 31; pQa = (Qa & 1u) << 31; pPb = (Pb & 1u) << 31; pQb = (Qb & 1u) << 31; }
+        if (lane == r) { mPa = Pa; mPb = Pb; }
+        if (TWO) {
+            const unsigned Qa = __ballot_sync(0xffffffffu, d.x < nm.hi), Qb = __ballot_sync(0xffffffffu, d.y < nm.hi);
+            if (lane == r) { mQa = Qa; mQb = Qb; }
+        }
         if (r >= Td::ROW0) {
             const int n0 = 32 * r;
-            const int nstart = FULL ? 1 : Td::NFIRST;
-            const unsigned valid = n0 >= nstart ? 0xffffffffu : (n0 + 32 <= nstart ? 0u : (0xffffffffu << (nstart - n0)));
-            const unsigned cPa = (Pa ^ __funnelshift_l(pPa, Pa, 1)) & valid, cPb = (Pb ^ __funnelshift_l(pPb, Pb, 1)) & valid;
-            fa += __popc(cPa); fb += __popc(cPb);
-            if (!FULL && r == Td::ROW0) { la += int((cPa >> Td::LANE0) & 1u); lb += int((cPb >> Td::LANE0) & 1u); }
-            if (TWO) {
-                const unsigned cQa = (Qa ^ __funnelshift_l(pQa, Qa, 1)) & valid, cQb = (Qb ^ __funnelshift_l(pQb, Qb, 1)) & valid;
-                fa += __popc(cQa); fb += __popc(cQb);
-                if (!FULL && r == Td::ROW0) { la += int((cQa >> Td::LANE0) & 1u); lb += int((cQb >> Td::LANE0) & 1u); }
-            }
             const float2 y = __ffma2_rn(a2, d, bp2);
             const bool live = !(r == Td::ROW0 && Td::LANE0 > 0) || lane >= Td::LANE0;
             const int b0 = (n0 / Lt) < 10 ? (n0 / Lt) : 10;
@@ -463,8 +465,12 @@ __device__ __forceinline__ void td_pair(const float2 (&u)[R], float cm, const b2
                 if (i1 >= 0 && i1 < Td::NE) { if (live && !first) e2[i1] = __ffma2_rn(y, y, e2[i1]); }
             }
         }
-        pPa = Pa; pQa = Qa; pPb = Pb; pQb = Qb;
     }
+    // both frames' counts in one reduction: a in bits 0..15, b in 16..31 (each field stays below 2^14)
+    unsigned v = td_row_flips<R, FULL>(mPa, lane) + (td_row_flips<R, FULL>(mPb, lane) << 16);
+    if (TWO) v += td_row_flips<R, FULL>(mQa, lane) + (td_row_flips<R, FULL>(mQb, lane) << 16);
+    v = __reduce_add_sync(0xffffffffu, v);
+    const int fa = int(v & 0xfffu), la = int((v >> 12) & 0xfu), fb = int((v >> 16) & 0xfffu), lb = int(v >> 28);
     flips_a = TWO ? fa : 2 * fa; link_a = TWO ? la : 2 * la;
     flips_b = TWO ? fb : 2 * fb; link_b = TWO ? lb : 2 * lb;
 }
@@ -621,7 +627,8 @@ __global__ void __launch_bounds__(32 * pair_warps<R>(), kPairMinBlocks) st_pair_
     const FeatTables ftab{t_dct, t_mrec, t_mw, t_chr, pp.pbl.lq, pp.pbl.ct};
     PairWarpMem<R> &wm = cm_.w[warp];
     float *const rowa = reinterpret_cast<float *>(wm.tz);
-    float *const t_re = reinterpret_cast<float *>(wm.tz), *const t_im = t_re + R * LS;
+    // this lane's slots in a pass-1 row (lane = n2)
+    const int t_re = 4 * (lane >> 1) + (lane & 1) + 2 * (lane >> 4), t_im = t_re ^ 2;
     float *const msraw = rowa + S::MS0, *const mslog = msraw + 2 * B200AA_N_MEL, *const mfold = mslog + 2 * B200AA_N_MEL;
     const int step = p.step;
     const int half = lane >> 4, l16 = lane & 15;
@@ -703,7 +710,8 @@ __global__ void __launch_bounds__(32 * pair_warps<R>(), kPairMinBlocks) st_pair_
                 if (is16) {
 #pragma unroll
                     for (int r = 0; r < R; ++r)
-                        uab[r] = make_float2(__int_as_float(0x4B000000 | (int(wa[r]) ^ 0x8000)), __int_as_float(0x4B000000 | (int(wb[r]) ^ 0x8000)));
+                        // wa / wb hold the 16-bit samples zero-extended: (x ^ 0x8000) | 0x4B000000 in one xor
+                        uab[r] = make_float2(__uint_as_float(wa[r] ^ 0x4B008000u), __uint_as_float(wb[r] ^ 0x4B008000u));
                 } else {
 #pragma unroll
                     for (int r = 0; r < R; ++r) uab[r] = make_float2(__int_as_float(wa[r]), __int_as_float(wb[r]));
@@ -824,11 +832,11 @@ __global__ void __launch_bounds__(32 * pair_warps<R>(), kPairMinBlocks) st_pair_
                 a_flat = !__any_sync(FULLM, zz.x > 0.f);
                 b_flat = !__any_sync(FULLM, zz.y > 0.f);
                 fft_r<R>(z);
-                t_re[lane] = z[0].x; t_im[lane] = z[0].y;
+                rowa[t_re] = z[0].x; rowa[t_im] = z[0].y;
 #pragma unroll
                 for (int k1 = 1; k1 < R; ++k1) {
                     const float2 w = cmul(z[k1], cm_.tw[k1 * 32 + lane]);
-                    t_re[k1 * LS + lane] = w.x; t_im[k1 * LS + lane] = w.y;
+                    rowa[k1 * LS + t_re] = w.x; rowa[k1 * LS + t_im] = w.y;
                 }
             }
             __syncwarp();
@@ -838,9 +846,14 @@ __global__ void __launch_bounds__(32 * pair_warps<R>(), kPairMinBlocks) st_pair_
                 {
                     float2 re[16], im[16];
                     const int row = lane < R ? lane : 0;
-                    const float2 *pr = reinterpret_cast<const float2 *>(t_re + row * LS), *pi = reinterpret_cast<const float2 *>(t_im + row * LS);
+                    const float4 *pq = reinterpret_cast<const float4 *>(rowa + row * LS);
 #pragma unroll
-                    for (int m = 0; m < 16; ++m) { re[m] = pr[m]; im[m] = pi[m]; }
+                    for (int m = 0; m < 16; ++m) {
+                        const float4 t = pq[m];
+                        const float2 lo = make_float2(t.x, t.y), hi = make_float2(t.z, t.w);
+                        re[m] = m < 8 ? lo : hi;
+                        im[m] = m < 8 ? hi : lo;
+                    }
                     fft32_soa(re, im, v);
                 }
                 __syncwarp();
