@@ -142,7 +142,8 @@ int b200aa_long_term_mean(const float *d_mid, int64_t n_clips, int n_rows, int64
 
 /* Feature vectors for the classifiers that consume the mid-term matrix (SURVEY 8f rank 4): d_out float32
  * [n_clips, n_windows, n_rows], vector j of clip b = (d_mid[b, :, j] - mean) / std -- the transpose the per-window loops
- * build one column at a time.  d_mean / d_std: float32 [n_rows] on the device.
+ * build one column at a time.  d_mean / d_std: float32 [n_rows] on the device.  Any number of clips; more than
+ * 65 535 * 32 rows returns B200AA_ERR_UNSUPPORTED.
  * Replaces: `feature_vector = (mt_feats[:, col_index] - mean) / std` per window (audioSegmentation.py:581-584,
  * audioTrainTest.py:1091) and per short-term frame (audioSegmentation.py:744-748, with d_mid = the [68 x T] matrix). */
 int b200aa_normalize_windows(const float *d_mid, int64_t n_clips, int n_rows, int64_t n_windows,

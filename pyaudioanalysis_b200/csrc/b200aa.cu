@@ -707,10 +707,17 @@ extern "C" int b200aa_normalize_windows(const float *d_mid, int64_t n_clips, int
 {
     if (!d_mid || !d_out || !d_mean || !d_std || n_clips < 0 || n_rows < 1 || n_windows < 0) return B200AA_ERR_INVALID;
     if (n_clips == 0 || n_windows == 0) return B200AA_OK;
-    if (n_clips > 65535 || (n_rows + 31) / 32 > 65535) return B200AA_ERR_UNSUPPORTED;
-    const dim3 grid((unsigned)((n_windows + 31) / 32), (unsigned)((n_rows + 31) / 32), (unsigned)n_clips), block(32, 8);
-    normalize_windows_kernel<<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(d_mid, n_rows, n_windows, d_mean, d_std, d_out);
-    CK_LAUNCH("normalize_windows_kernel");
+    if ((n_rows + 31) / 32 > 65535) return B200AA_ERR_UNSUPPORTED;
+    // grid.z holds at most 65 535 clips: larger batches run as slabs of that many, each offset by whole clips
+    constexpr int64_t kSlab = 65535;
+    const size_t clip_elems = size_t(n_rows) * size_t(n_windows);
+    for (int64_t b0 = 0; b0 < n_clips; b0 += kSlab) {
+        const int64_t nb = std::min<int64_t>(kSlab, n_clips - b0);
+        const dim3 grid((unsigned)((n_windows + 31) / 32), (unsigned)((n_rows + 31) / 32), (unsigned)nb), block(32, 8);
+        normalize_windows_kernel<<<grid, block, 0, static_cast<cudaStream_t>(stream)>>>(
+            d_mid + size_t(b0) * clip_elems, n_rows, n_windows, d_mean, d_std, d_out + size_t(b0) * clip_elems);
+        CK_LAUNCH("normalize_windows_kernel");
+    }
     return B200AA_OK;
 }
 

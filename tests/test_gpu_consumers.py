@@ -19,22 +19,6 @@ def P():
     return pkg
 
 
-def test_normalize_windows_kernel(P):
-    import torch
-    from pyaudioanalysis_b200.consumers import normalize_windows_batch
-    rng = np.random.default_rng(11)
-    for B, F, M in ((1, 136, 8), (3, 136, 77), (2, 68, 399), (5, 7, 1), (1, 33, 65)):
-        mid = rng.normal(size=(B, F, M)).astype(np.float32)
-        mean = rng.normal(size=F)
-        std = rng.uniform(0.5, 2.0, size=F)
-        out = normalize_windows_batch(torch.from_numpy(mid).cuda(), mean, std).cpu().numpy()
-        ref = ((mid.astype(np.float64) - mean[None, :, None]) / std[None, :, None]).transpose(0, 2, 1)
-        assert out.shape == (B, M, F)
-        assert np.allclose(out, ref, rtol=2e-6, atol=2e-6)
-    with pytest.raises(ValueError):
-        normalize_windows_batch(torch.zeros((1, 4, 4), device="cuda"), np.zeros(3), np.ones(3))
-
-
 def test_mid_term_classification_matches_reference_loop(P):
     """Windows of a two-part clip (noise, then a tone) through mid features -> normalise -> SVM / kNN: labels and maximum
     posteriors of the batched path equal the reference's per-window loop run on the oracle's float64 matrix."""

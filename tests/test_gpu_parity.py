@@ -342,15 +342,6 @@ def test_host_pipeline(P):
     check_features(got2[3], O.feature_extraction(big[3], 16000, 800, 400)[0], 400, "chunked host pipeline clip 3")
 
 
-def test_mid_pool_kernel(P):
-    import torch
-    from pyaudioanalysis_b200.batch import mid_pool_batch
-    st = torch.randn(3, 68, 399, device="cuda")
-    mid = mid_pool_batch(st, 39, 40).cpu().numpy()
-    ref = np.stack([O.mid_pool(st[i].cpu().numpy().astype(np.float64), 39, 40) for i in range(3)])
-    check_close(mid, ref, "mid_pool", rtol=1e-5, atol=1e-6)
-
-
 def test_kernel_kinds_agree(P):
     """Every kernel that exists for a window (2 = warp-autonomous pair kernel, 3 = warp-autonomous per-frame ("solo") kernel,
     1 = register-tiled CTA kernel, 0 = generic) must agree with the oracle; the default plan picks the fastest one."""
